@@ -52,7 +52,20 @@ def parse_args():
                     help="weak: every rank gets the workload's pockets (default for c2/c3/c1); strong: ONE global batch is "
                          'partitioned over the ranks by atom count (default for c5: 256 ragged pockets over the box)')
     ap.add_argument('--global-graphs', type=int, default=None, help='pockets of the global batch for --scaling strong')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the ligand state the last timed step computed (coordinates x_lig '
+                         '[n_lig, 3] and atom-type one-hots c_lig [n_lig, K], float32) as DIR/<name>.npy; the inputs are '
+                         'seeded, so two builds run with the same arguments can be compared output for output')
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """Write each device tensor as out_dir/<name>.npy (float32); with several ranks every rank writes <name>.rank<r>.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = '' if world == 1 else f'.rank{rank}'
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f'{name}{suffix}.npy'), t.detach().float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------
@@ -241,6 +254,8 @@ def run_b200(args):
     assert world == args.gpus, f'--gpus {args.gpus} but WORLD_SIZE={world} (launch N>1 with torchrun)'
     if args.warmup < 3:
         raise SystemExit('--warmup must be >= 3')
+    if args.steps < 1:
+        raise SystemExit('--steps must be >= 1')
     dev = torch.device('cuda', local_rank)
     torch.cuda.set_device(dev)
     torch.set_grad_enabled(False)
@@ -300,6 +315,9 @@ def run_b200(args):
             ends[i].record()
         barrier()
     gpu_launches = L.cbg_launch_count() - launches0
+    if args.dump_outputs:
+        t_out = t_seq[args.warmup + args.steps - 1]        # slot t of X / Cc holds the result of step t
+        dump_outputs(args.dump_outputs, {'x_lig': X[t_out], 'c_lig': Cc[t_out]}, rank, world)
     step_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     ms_per_step = sum(step_ms) / len(step_ms)
     t = torch.tensor([ms_per_step], device=dev, dtype=torch.float64)

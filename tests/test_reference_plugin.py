@@ -1,114 +1,61 @@
-"""The drop-in seams on the REAL reference (INTEGRATION.md section 2), on the GPU box: the staged copy of the reference
-(baseline/_ref, see baseline/ref_runner.py) is imported unmodified, the ~15-line plugin is applied, and
+"""The drop-in seams of INTEGRATION.md section 2, against what the UNMODIFIED reference computes on the same inputs
+(tests/golden/plugin_seam.npz, written by tests/golden/make_golden_plugin.py from the reference's own
+``TargetDiff.sample`` with its own denoiser and injected noise):
 
-* seam 1: the reference's own ``TargetDiff`` (its sample() loop, its embedder, its schedulers) runs with
-  ``UniTransformerB200`` as the denoiser (``get_e3_gnn`` patched) - same checkpoint keys, same trajectory;
-* seam 2: ``get_model(cfg)`` returns ``TargetDiffB200`` for the reference's EasyDict config and loads the same state dict.
+* seam 1: ``UniTransformerB200`` (what the patched ``get_e3_gnn`` returns) is called exactly the way the reference's
+  sample loop calls its denoiser - ``denoiser(batch_idx=..., x=..., h=..., gen_flag=..., lig_flag=...)`` -> ``(x, h, v)``,
+  with the arguments recorded from the loop's first step - and returns the reference denoiser's outputs;
+* seam 2: ``get_model(cfg)`` returns ``TargetDiffB200`` for the reference's EasyDict config, loads the same state dict and
+  samples the reference's trajectory.
 
-Both are checked against the oracle with injected noise (atom types bit-exact, coordinates within 1e-4)."""
-import sys
-
+Atom types bit-exact, coordinates within 1e-4 of the reference and of the oracle."""
+import numpy as np
 import pytest
 import torch
 
 from cbgbench_b200 import synthetic
-from helpers import assert_close, make_model, rel_err
+from helpers import assert_close, golden, make_model, rel_err
 
 pytestmark = pytest.mark.gpu
 torch.set_grad_enabled(False)
-
-
-def _reference():
-    from baseline import ref_runner
-    if ref_runner.ref_root() is None:
-        pytest.skip('no staged reference (baseline/_ref) and no /root/reference')
-    ref_runner.install()
-    return ref_runner
-
-
-def _apply_plugin():
-    """INTEGRATION.md section 2, verbatim in spirit: patch the two factories BEFORE the model modules bind them."""
-    import repo.modules.e3nn as e3nn
-    import repo.models._base as model_registry
-    from cbgbench_b200 import UniTransformerB200, TargetDiffB200
-    if not hasattr(e3nn, '_orig_get_e3_gnn'):
-        e3nn._orig_get_e3_gnn = e3nn.get_e3_gnn
-
-    def get_e3_gnn(cfg, num_classes=None, num_edge_classes=None):
-        if cfg.type == 'unitransformer':
-            if num_classes is not None:
-                cfg.num_classes = num_classes
-            return UniTransformerB200(cfg)
-        return e3nn._orig_get_e3_gnn(cfg, num_classes, num_edge_classes)
-
-    e3nn.get_e3_gnn = get_e3_gnn
-    if 'repo.models.diffusion.targetdiff' in sys.modules:      # already imported in this process: rebind its name too
-        sys.modules['repo.models.diffusion.targetdiff'].get_e3_gnn = get_e3_gnn
-    import repo.models.diffusion.targetdiff as tdm
-    model_registry._MODEL_DICT['targetdiff_ref_loop'] = tdm.TargetDiff     # the reference's own class, for seam 1
-    model_registry._MODEL_DICT['targetdiff'] = TargetDiffB200
-    return e3nn, model_registry, tdm
-
-
-def _inject_noise(pn, tu, T):
-    calls = {'randn': 0, 'rand': 0}
-    orig = (torch.randn_like, torch.rand_like)
-
-    def fake_randn_like(a, *aa, **kk):      # once per step, t = T-1 ... 0 (diffusion_scheduler.py:163)
-        t = T - 1 - calls['randn']
-        calls['randn'] += 1
-        return pn[t].to(a.device)
-
-    def fake_rand_like(a, *aa, **kk):       # categorical.py:27
-        t = T - 1 - calls['rand']
-        calls['rand'] += 1
-        return tu[t].to(a.device)
-
-    torch.randn_like, torch.rand_like = fake_randn_like, fake_rand_like
-    return orig, calls
+TOL = 1e-4
+# must match tests/golden/make_golden_plugin.py
+T = 6
+N_PROT, N_LIG = [120, 70], [14, 9]
+DATA_SEED, NOISE_SEED = 61, 17
 
 
 def test_reference_sample_loop_with_b200_denoiser_and_get_model_seam():
+    from baseline import ref_runner
+    from cbgbench_b200 import TargetDiffB200, UniTransformerB200, get_model
     from oracle import diffusion as OD
-    rr = _reference()
-    e3nn, registry, tdm = _apply_plugin()
-    T = 6
+    g = golden('plugin_seam.npz')
     dev = torch.device('cuda:0')
     _, sd = make_model(T)
-    batch = synthetic.make_batch([120, 70], [14, 9], seed=61)
-    n_lig = 23
-    pn, tu = synthetic.make_noise(T, n_lig, 13, seed=17)
+    batch = synthetic.make_batch(N_PROT, N_LIG, seed=DATA_SEED)
+    pn, tu = synthetic.make_noise(T, sum(N_LIG), 13, seed=NOISE_SEED)
     want = OD.sample(sd, batch, T, pn, tu)
-    dbatch = {k: (v.to(dev) if torch.is_tensor(v) else v) for k, v in batch.items()}
-
-    # ---- seam 1: reference TargetDiff.sample, B200 denoiser inside
-    cfg = rr.targetdiff_cfg(T)
-    cfg.type = 'targetdiff_ref_loop'
-    ref = registry.get_model(cfg)
-    from cbgbench_b200 import UniTransformerB200
-    assert type(ref) is tdm.TargetDiff and isinstance(ref.denoiser, UniTransformerB200)
-    ref.load_state_dict(sd, strict=True)                       # identical keys / shapes
-    ref = ref.to(dev).eval()
-    tdm.tqdm = lambda it, **kw: it
-    orig, calls = _inject_noise(pn, tu, T)
-    try:
-        traj = ref.sample(dbatch)
-    finally:
-        torch.randn_like, torch.rand_like = orig
-    assert calls == {'randn': T, 'rand': T}
-    for t in range(-1, T - 1):
-        xg, cg = traj[t][0].cpu(), traj[t][1].cpu()
-        assert torch.equal(cg.argmax(-1), want[t][1].argmax(-1)), t
-        assert rel_err(xg, want[t][0]) < 1e-4, (t, rel_err(xg, want[t][0]))
-        assert_close(xg, want[t][0], rtol=1e-4, atol=1e-5, what=f'seam 1 x t={t}')
 
     # ---- seam 2: get_model(cfg) -> TargetDiffB200 built from the reference's EasyDict config
-    from cbgbench_b200 import TargetDiffB200
-    mine = registry.get_model(rr.targetdiff_cfg(T))
-    assert isinstance(mine, TargetDiffB200)
-    mine.load_state_dict(sd, strict=True)
+    mine = get_model(ref_runner.targetdiff_cfg(T))
+    assert isinstance(mine, TargetDiffB200) and isinstance(mine.denoiser, UniTransformerB200)
+    mine.load_state_dict(sd, strict=True)                      # identical keys / shapes
     mine = mine.to(dev).eval()
-    traj2 = mine.sample(dbatch, pos_noise=pn, type_uniform=tu)
+
+    # ---- seam 1: the denoiser call of the reference's sample loop, keyword for keyword
+    call = {k[len('call/in/'):]: torch.from_numpy(g[k]).to(dev) for k in g.files if k.startswith('call/in/')}
+    assert sorted(call) == ['batch_idx', 'gen_flag', 'h', 'lig_flag', 'x']
+    x, h, v = mine.denoiser(**call)
+    for got, k in ((x, 'x'), (h, 'h'), (v, 'v')):
+        assert rel_err(got.cpu(), g[f'call/out/{k}']) < TOL, (k, rel_err(got.cpu(), g[f'call/out/{k}']))
+    assert_close(x.cpu(), g['call/out/x'], rtol=1e-4, atol=1e-4, what='seam 1 denoiser x')
+
+    dbatch = {k: (v_.to(dev) if torch.is_tensor(v_) else v_) for k, v_ in batch.items()}
+    traj = mine.sample(dbatch, pos_noise=pn, type_uniform=tu)
     for t in range(-1, T - 1):
-        assert torch.equal(traj2[t][1].cpu().argmax(-1), want[t][1].argmax(-1)), t
-        assert rel_err(traj2[t][0].cpu(), want[t][0]) < 1e-4, t
+        xg, vg = traj[t][0].cpu(), traj[t][1].cpu().argmax(-1)
+        assert np.array_equal(vg.numpy(), g[f'v{t}'].astype(np.int64)), t
+        assert torch.equal(vg, want[t][1].argmax(-1)), t
+        assert rel_err(xg, g[f'x{t}']) < TOL, (t, rel_err(xg, g[f'x{t}']))
+        assert_close(xg, g[f'x{t}'], rtol=1e-4, atol=1e-5, what=f'seam 2 x t={t}')
+        assert rel_err(xg, want[t][0]) < TOL, (t, rel_err(xg, want[t][0]))
