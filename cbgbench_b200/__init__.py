@@ -6,6 +6,7 @@ Only what the path needs (DESIGN.md):
   targetdiff.py TargetDiff.sample drop-in (outer diffusion loop in Python, one C call per step)
   diffsbdd.py   DiffSBDD.sample drop-in (row f2: variational schedule + COM projection on the same denoiser)
   diffbp.py     DiffBP.sample drop-in (row f2: CoM head = 3 more H2X layers, score-form VP step, mask-type step)
+  difffg.py     D3FG.sample drop-in (FG context embedder, IPA encoder, position / SO(3) / FG-type reverse step)
   schedulers.py noise-schedule tables (checkpoint-compatible parameter containers)
   sharding.py   pocket sharding over GPUs + the single gather of final coordinates
   batch_builder.py  sampling batches built on the GPU from raw pockets (row f3: size prior, types, positions, collate)
@@ -18,6 +19,7 @@ from .modules import UniTransformerB200, get_e3_gnn  # noqa: F401
 from .targetdiff import TargetDiffB200, get_model, register_model  # noqa: F401
 from .diffsbdd import DiffSBDDB200  # noqa: F401
 from .diffbp import DiffBPB200  # noqa: F401
+from .difffg import D3FGB200  # noqa: F401
 from .batch_builder import DeviceBatchBuilder, SizePrior  # noqa: F401
 
 __version__ = '0.1.0'

@@ -42,6 +42,26 @@ class BpCoef(C.Structure):
     _fields_ = [('alpha_cumprod', C.c_float), ('beta', C.c_float), ('nonzero', C.c_float), ('change_prob', C.c_float)]
 
 
+class D3fgPlan(C.Structure):
+    _fields_ = [
+        ('blob', C.c_void_p), ('hidden', C.c_int32), ('num_sublayers', C.c_int32), ('num_blocks', C.c_int32),
+        ('num_classes', C.c_int32), ('k', C.c_int32), ('graph_ptr', C.c_void_p), ('n_graphs', C.c_int32),
+        ('max_graph_nodes', C.c_int32), ('n_nodes', C.c_int64), ('lig_flag', C.c_void_p), ('gen_flag', C.c_void_p),
+        ('lig_node', C.c_void_p), ('n_lig', C.c_int32), ('gen_lig', C.c_void_p), ('fg_wt', C.c_void_p), ('fg_b', C.c_void_p),
+        ('lig_bias', C.c_void_p), ('h_static', C.c_void_p), ('x', C.c_void_p), ('o', C.c_void_p), ('rot_cdf', C.c_void_p),
+        ('rot_x', C.c_void_p), ('n_bins', C.c_int32), ('workspace', C.c_void_p), ('workspace_bytes', C.c_int64),
+    ]
+
+
+class D3fgCoef(C.Structure):
+    _fields_ = [
+        ('alpha_cumprod', C.c_float), ('beta', C.c_float), ('pos_nonzero', C.c_float),
+        ('rot_stddev', C.c_float), ('rot_approx', C.c_int32), ('rot_nonzero', C.c_float), ('rot_row', C.c_int32),
+        ('log_alphas_cumprod_prev', C.c_float), ('log_one_minus_alphas_cumprod_prev', C.c_float),
+        ('log_alpha', C.c_float), ('log_one_minus_alpha', C.c_float),
+    ]
+
+
 _P, _I32, _I64, _F, _SZ = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
 
 # name -> (restype, argtypes); must list every symbol of include/cbg_b200.h
@@ -96,6 +116,9 @@ SIGNATURES = {
     'cbg_ipa_workspace_bytes': (_I64, [_I64, _I32]),
     'cbg_ipa_forward_f32': (_I32, [_P, _I32, _I32, _I32, _I32, _P, _P, _P, _P, _I32, _I32, _P, _P, _I64, _I32,
                                    _P, _P, _P, _P, _P, _P, _I64, _P]),
+    'cbg_d3fg_workspace_bytes': (_I64, [_I64, _I32, _I32]),
+    'cbg_d3fg_step_f32': (_I32, [C.POINTER(D3fgPlan), C.POINTER(D3fgCoef)] + [_P] * 17),
+    'cbg_d3fg_reverse_f32': (_I32, [C.POINTER(D3fgCoef), _P, _P, _I32] + [_P] * 13 + [_I32, _I32] + [_P] * 6),
     'cbg_reverse_step_f32': (_I32, [C.POINTER(StepCoef), _P, _P, _P, _P, _P, _P, _P, _I32, _I32, _P, _P, _P, _P]),
 }
 

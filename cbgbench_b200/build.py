@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_PATH = os.path.join(HERE, 'libcbg_b200.so')
-SOURCES = ['api.cu', 'graph.cu', 'node_gemm.cu', 'node_gemm_tc.cu', 'node_gemm_f16.cu', 'edge.cu', 'x2h_tc.cu', 'misc.cu', 'batch.cu', 'ipa.cu']
+SOURCES = ['api.cu', 'graph.cu', 'node_gemm.cu', 'node_gemm_tc.cu', 'node_gemm_f16.cu', 'edge.cu', 'x2h_tc.cu', 'misc.cu', 'batch.cu', 'ipa.cu', 'd3fg.cu']
 HEADERS = ['cbg_common.cuh', 'cbg_kernels.cuh', 'cbg_layout.h', 'cbg_tc.cuh', '../../include/cbg_b200.h']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-shared']

@@ -215,3 +215,12 @@ int cbg_launch_build_batch(const float* prot_pos, const int* prot_element, const
                            float* o_prot_pos, float* o_prot_feat, long long* o_prot_aa, long long* o_prot_batch,
                            float* o_prot_tr, float* o_lig_pos, long long* o_lig_type, long long* o_lig_batch,
                            unsigned char* o_lig_ctx, unsigned char* o_lig_gen, cudaStream_t st);
+
+// ipa.cu (row f4: D3FG encoder).  The head block has its own class bound: D3FG's fg_only mode has 28 FG types, while the
+// denoiser blob (cbg_layout.h) keeps CBG_MAXCLS.
+#define CBG_IPA_MAXCLS 32
+// h_out == h_in: the layers update h in place (no copy); ws: cbg_ipa_workspace_bytes(n_nodes, hidden), 256-byte aligned
+int cbg_launch_ipa_forward(const float* blob, int hidden, int num_sublayers, int num_blocks, int num_classes, const float* x,
+                           const float* o, const float* h_in, const int* graph_ptr, int n_graphs, int max_graph_nodes,
+                           const unsigned char* lig_flag, const unsigned char* gen_flag, int n_nodes, int k, float* eps_pos,
+                           float* h_out, float* o_next, float* r_next, float* logits, char* ws, cudaStream_t st);

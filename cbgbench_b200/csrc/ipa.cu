@@ -31,8 +31,8 @@ __host__ __device__ inline long long head_size(int H, int f) {
     case IH_ROT_B2: case IH_CRD_B2: return 4;
     case IH_CLS_W0T: return (long long)H * H;
     case IH_CLS_B0: return H;
-    case IH_CLS_W1: return CBG_MAXCLS * H;
-    case IH_CLS_B1: return CBG_MAXCLS;
+    case IH_CLS_W1: return CBG_IPA_MAXCLS * H;
+    case IH_CLS_B1: return CBG_IPA_MAXCLS;
   }
   return 0;
 }
@@ -407,6 +407,17 @@ int ipa_forward_t(const float* blob, int num_sublayers, int num_blocks, int num_
 
 }  // namespace
 
+int cbg_launch_ipa_forward(const float* blob, int hidden, int num_sublayers, int num_blocks, int num_classes, const float* x,
+                           const float* o, const float* h_in, const int* graph_ptr, int n_graphs, int max_graph_nodes,
+                           const unsigned char* lig_flag, const unsigned char* gen_flag, int n_nodes, int k, float* eps_pos,
+                           float* h_out, float* o_next, float* r_next, float* logits, char* ws, cudaStream_t st) {
+  if (hidden == 128)
+    return ipa_forward_t<128>(blob, num_sublayers, num_blocks, num_classes, x, o, h_in, graph_ptr, n_graphs, max_graph_nodes,
+                              lig_flag, gen_flag, n_nodes, k, eps_pos, h_out, o_next, r_next, logits, ws, st);
+  return ipa_forward_t<256>(blob, num_sublayers, num_blocks, num_classes, x, o, h_in, graph_ptr, n_graphs, max_graph_nodes,
+                            lig_flag, gen_flag, n_nodes, k, eps_pos, h_out, o_next, r_next, logits, ws, st);
+}
+
 extern "C" {
 
 int64_t cbg_ipa_head_floats(int32_t hidden) {
@@ -447,17 +458,14 @@ int32_t cbg_ipa_forward_f32(const float* blob, int32_t hidden, int32_t num_subla
                             int32_t k, float* eps_pos, float* h_out, float* o_next, float* r_next, float* logits,
                             void* workspace, int64_t workspace_bytes, void* stream) {
   if (hidden != 128 && hidden != 256) { cbg_set_error("cbg_ipa_forward_f32: hidden=%d (128 or 256)", hidden); return 1; }
-  if (num_classes < 1 || num_classes > CBG_MAXCLS) { cbg_set_error("num_classes=%d outside [1,%d]", num_classes, CBG_MAXCLS); return 1; }
+  if (num_classes < 1 || num_classes > CBG_IPA_MAXCLS) { cbg_set_error("num_classes=%d outside [1,%d]", num_classes, CBG_IPA_MAXCLS); return 1; }
   if (n_nodes <= 0 || n_nodes > 0x7fffffffLL / (5 * 256)) { cbg_set_error("n_nodes=%lld out of range", (long long)n_nodes); return 1; }
   if (!workspace || workspace_bytes < cbg_ipa_workspace_bytes(n_nodes, hidden)) { cbg_set_error("workspace too small"); return 1; }
   if (((uintptr_t)workspace & 255) != 0) { cbg_set_error("workspace must be 256-byte aligned"); return 1; }
   if (num_blocks < 1 || num_sublayers < 0) { cbg_set_error("num_blocks / num_sublayers"); return 1; }
-  cudaStream_t st = (cudaStream_t)stream;
-  if (hidden == 128)
-    return ipa_forward_t<128>(blob, num_sublayers, num_blocks, num_classes, x, o, h, graph_ptr, n_graphs, max_graph_nodes,
-                              lig_flag, gen_flag, (int)n_nodes, k, eps_pos, h_out, o_next, r_next, logits, (char*)workspace, st);
-  return ipa_forward_t<256>(blob, num_sublayers, num_blocks, num_classes, x, o, h, graph_ptr, n_graphs, max_graph_nodes,
-                            lig_flag, gen_flag, (int)n_nodes, k, eps_pos, h_out, o_next, r_next, logits, (char*)workspace, st);
+  return cbg_launch_ipa_forward(blob, hidden, num_sublayers, num_blocks, num_classes, x, o, h, graph_ptr, n_graphs,
+                                max_graph_nodes, lig_flag, gen_flag, (int)n_nodes, k, eps_pos, h_out, o_next, r_next, logits,
+                                (char*)workspace, (cudaStream_t)stream);
 }
 
 }  // extern "C"

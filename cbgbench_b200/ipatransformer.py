@@ -16,6 +16,8 @@ from . import _lib
 from .modules import (GaussianSmearing, MLP, ShiftedSoftplus, _NoTorchPath, _Workspace, cfg_get, graph_ptr_from_batch,
                       N_HEADS, N_RBF)
 
+MAX_CLASSES = 32      # CBG_IPA_MAXCLS (csrc/cbg_kernels.cuh): D3FG's fg_only mode has 28 FG types
+
 
 class X2HAttentionW(_NoTorchPath):
     """Parameters of x2h_attention.py:8-41 at hidden width ``hidden`` (ew_net_type='global', out_fc=False)."""
@@ -90,7 +92,7 @@ def pack_ipa_blob(sd, hidden, num_layers, num_x2h, num_classes):
         put(g0, head_f, f'{tag}_B2', t(f'{net}.4.bias'))
     put(g0, head_f, 'CLS_W0T', t('classifier.0.weight').t().contiguous())
     put(g0, head_f, 'CLS_B0', t('classifier.0.bias'))
-    assert t('classifier.2.weight').shape == (num_classes, hidden) and num_classes <= 16
+    assert t('classifier.2.weight').shape == (num_classes, hidden) and num_classes <= MAX_CLASSES
     put(g0, head_f, 'CLS_W1', t('classifier.2.weight'))
     put(g0, head_f, 'CLS_B1', t('classifier.2.bias'))
     inv = 1.0 / math.sqrt(hidden // N_HEADS)
@@ -159,8 +161,8 @@ class IPATransformerB200(nn.Module):
             unsupported.append(f'cutoff_mode={self.cutoff_mode}')
         if not (1 <= self.cut_off <= 32):
             unsupported.append('k outside [1,32]')
-        if self.num_classes is None or not (1 <= self.num_classes <= 16):
-            unsupported.append('num_classes must be in [1,16]')
+        if self.num_classes is None or not (1 <= self.num_classes <= MAX_CLASSES):
+            unsupported.append(f'num_classes must be in [1,{MAX_CLASSES}]')
         if unsupported:
             raise NotImplementedError('IPATransformerB200: unsupported configuration: ' + ', '.join(unsupported))
         H = self.hidden_dim

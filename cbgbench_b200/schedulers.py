@@ -1,4 +1,4 @@
-"""Noise-schedule tables of the reference's TargetDiff path, as parameter containers.
+"""Noise-schedule tables of the reference's diffusion models, as parameter containers.
 
 Mirrors the state-dict layout of ``VPScheduler`` / ``CTNVPScheduler`` / ``TypeVPScheduler``
 (/root/reference repo/models/diffusion/diffusion_scheduler.py:27-100, 102-165, 320-337): every
@@ -6,6 +6,8 @@ table is a frozen fp32 ``nn.Parameter`` under the reference's name, so checkpoin
 unchanged (the tables ARE checkpointed, SURVEY.md a15).  The reverse steps themselves run in
 the fused CUDA step (csrc/misc.cu: reverse_kernel); this file only builds tables.
 """
+import math
+
 import numpy as np
 import torch
 from torch import nn
@@ -94,6 +96,63 @@ class TypeVPTables(VPTables):
         self.log_one_minus_alphas_v = _frozen(one_minus(log_a))
         self.log_alphas_cumprod_v = _frozen(log_acp)
         self.log_one_minus_alphas_cumprod_v = _frozen(one_minus(log_acp))
+
+
+# ---- D3FG: SO(3) rotation schedule ------------------------------------------------------------------------------------
+
+def angular_histogram(stddev, num_bins=8192, num_terms=1024):
+    """Bin edges X and unnormalised density Y of the isotropic Gaussian on SO(3) over the rotation angle, truncated
+    after ``num_terms`` terms of its series (ApproxAngularDistribution._pdf / _precompute_histograms, so3.py:82-109).
+    fp32 torch in the reference's operation order, so the rows are bit-equal to the reference's on the same build."""
+    x = torch.linspace(0, math.pi, num_bins)
+    xc = x[:, None]
+    l = torch.arange(0, num_terms)[None, :]
+    weight = (2 * l + 1) * torch.exp(-l * (l + 1) * (stddev ** 2))
+    ratio = (torch.sin((l + 0.5) * xc) + 1e-6) / (torch.sin(xc / 2) + 1e-6)
+    density = (((1 - torch.cos(xc)) / math.pi) * weight * ratio).sum(dim=1)
+    return x, torch.nan_to_num(density).clamp_min(0)
+
+
+class AngularDistributionTables(nn.Module):
+    """Buffers of ApproxAngularDistribution (so3.py:71-109): stddevs [T], approx_flag [T] (stddev <= 0.1: the sampler
+    uses the Gaussian approximation), X / Y [T, num_bins] (one histogram per stddev)."""
+
+    def __init__(self, stddevs, std_threshold=0.1, num_bins=8192, num_terms=1024):
+        super().__init__()
+        self.register_buffer('stddevs', torch.tensor(stddevs, dtype=torch.float32))
+        self.register_buffer('approx_flag', self.stddevs <= std_threshold)
+        rows = [angular_histogram(sd.item(), num_bins, num_terms) for sd in self.stddevs]
+        self.register_buffer('X', torch.stack([r[0] for r in rows]))
+        self.register_buffer('Y', torch.stack([r[1] for r in rows]))
+
+
+def rot_stddevs(alphas_cumprod, betas):
+    """(forward, inverse) stddev vectors of RotVPScheduler (diffusion_scheduler.py:514-527), fp32 like the reference:
+    forward sqrt(1 - abar_t); inverse sqrt((1 - abar_{t-1}) / (1 - abar_t) * beta_t), 0 at t = 0."""
+    fwd = torch.sqrt(1 - alphas_cumprod)
+    var = torch.zeros_like(betas)
+    for i in range(1, betas.shape[0]):
+        var[i] = ((1 - alphas_cumprod[i - 1]) / (1 - alphas_cumprod[i])) * betas[i]
+    return fwd.tolist(), torch.sqrt(var).tolist()
+
+
+class RotVPTables(VPTables):
+    """Orientation schedule (RotVPScheduler, diffusion_scheduler.py:514-529): the 12 VP tables, ``_dummy`` and the
+    histograms of the forward / inverse angular distributions under the reference's state-dict names.  Building the
+    histograms costs about 33 ms per stddev on 8 CPU threads (about a minute at T = 1000), as in the reference."""
+
+    def __init__(self, num_timestep, beta_start=1e-7, beta_end=2e-3, type='sigmoid', cosine_s=0.008):
+        super().__init__(num_timestep, beta_start, beta_end, type, cosine_s)
+        with torch.no_grad():
+            fwd, inv = rot_stddevs(self.alphas_cumprod.detach(), self.betas.detach())
+        self.angular_distrib_fwd = AngularDistributionTables(fwd)
+        self.angular_distrib_inv = AngularDistributionTables(inv)
+        self.register_buffer('_dummy', torch.empty([0]))
+
+    def inverse_cdf(self):
+        """float64 [T, num_bins - 1] = cumsum(angular_distrib_inv.Y[t, :-1]): the table the sampler's multinomial draw
+        searches (include/cbg_b200.h, DESIGN.md section 13)."""
+        return torch.cumsum(self.angular_distrib_inv.Y[:, :-1].detach().to('cpu', torch.float64), dim=1)
 
 
 # ---- DiffSBDD: variational gamma schedule (SURVEY.md section 8 row f2) ---------------------------------------

@@ -220,3 +220,110 @@ def make_ipa_inputs(hidden, n_nodes, n_lig, seed, gen_mode='denovo'):
         gens.append(gen)
     cat = lambda a, dt: torch.from_numpy(np.concatenate(a, 0).astype(dt))
     return (cat(xs, np.float32), cat(os_, np.float32), cat(hs, np.float32), cat(bs, np.int64), cat(ligs, bool), cat(gens, bool))
+
+
+# ---- D3FG sampler -----------------------------------------------------------------------------------------------------------
+# schedule tables (betas ... Y) and the fixed angular-encoding frequencies are not weights
+D3FG_SKIP = ('pos_scheduler.', 'rot_scheduler.', 'type_scheduler.', 'context_embedder.residue_emb.dihed_embed.')
+
+
+def d3fg_config(num_steps=1000, hidden=256, num_layers=9, num_fgtype=28):
+    """configs/denovo/train/d3fg_fg.yml:1-28 (+ num_fgtype: fg_only mode, configuration.py:6-10, 65).  The encoder type
+    is spelled 'ipatransformer', the name the reference's factory accepts (both spellings build the same module here)."""
+    return Cfg(dict(
+        type='difffg', num_fgtype=num_fgtype,
+        encoder=dict(type='ipatransformer', node_feat_dim=hidden, n_heads=16, num_layers=num_layers),
+        generator=dict(pos_schedule=dict(type='sigmoid', beta_start=1.e-7, beta_end=2.e-3),
+                       rot_schedule=dict(type='cosine', cosine_s=0.01), fg_schedule=dict(type='cosine', cosine_s=0.01),
+                       num_diffusion_timesteps=num_steps, time_sampler='symmetric'),
+        embedder=dict(type='fg', emb_dim=hidden, fg=dict(type='linear'), residue=dict(type='frame'))))
+
+
+def _random_so3vec(rs, n):
+    """so3 vectors of rotations uniform on SO(3) (unit quaternions from normalised Gaussians)."""
+    q = rs.normal(size=(n, 4))
+    q /= np.linalg.norm(q, axis=1, keepdims=True)
+    q[q[:, 0] < 0] *= -1
+    v = q[:, 1:]
+    s = np.linalg.norm(v, axis=1, keepdims=True)
+    theta = 2 * np.arctan2(s[:, 0], q[:, 0])
+    return v / np.maximum(s, 1e-12) * theta[:, None]
+
+
+def make_fg_batch(n_res, n_fg, seed=2024, gen_mode='denovo', num_fgtype=28):
+    """Flat D3FG sampling batch with the reference's keys (difffg.py:175-197): per graph ``n_res`` residues with
+    non-degenerate N / CA / C backbones (15 heavy-atom slots, side chains of random length), ragged chains with gaps in
+    the residue numbering, and ``n_fg`` functional groups with Gaussian centres, random types and orientations uniform
+    on SO(3).  gen_mode 'partial': the first third of every graph's FGs is fixed context (no ligand_gen_flag)."""
+    rs = np.random.RandomState(seed)
+    n_res, n_fg = list(n_res), list(n_fg)
+    assert len(n_res) == len(n_fg)
+    keys = ('pp', 'pm', 'aa', 'rnb', 'cnb', 'nch', 'lp', 'lo', 'lt', 'gen', 'bl', 'br')
+    acc = {k: [] for k in keys}
+    for g, (nr, nf) in enumerate(zip(n_res, n_fg)):
+        ca = np.cumsum(rs.normal(0.0, 2.2, size=(nr, 3)), axis=0)
+        ca -= ca.mean(0, keepdims=True)
+        pos = np.zeros((nr, 15, 3))
+        mask = np.zeros((nr, 15), dtype=bool)
+        for d, length in ((0, 1.46), (2, 1.52), (3, 2.4)):          # N, C, O around CA
+            u = rs.normal(size=(nr, 3))
+            pos[:, d] = ca + length * u / np.linalg.norm(u, axis=1, keepdims=True)
+        pos[:, 1] = ca
+        mask[:, :4] = True
+        n_side = rs.randint(0, 11, size=nr)
+        for r in range(nr):
+            pos[r, 4:4 + n_side[r]] = ca[r] + rs.normal(0.0, 1.5, size=(n_side[r], 3))
+            mask[r, 4:4 + n_side[r]] = True
+        acc['pp'].append(pos)
+        acc['pm'].append(mask)
+        acc['aa'].append(rs.randint(0, 20, size=nr))
+        acc['rnb'].append(1 + np.cumsum(rs.choice([1, 1, 1, 1, 2], size=nr)))
+        chains = 2 if nr >= 8 and g % 2 == 0 else 1
+        acc['cnb'].append((np.arange(nr) >= nr // 2).astype(np.int64) if chains == 2 else np.zeros(nr, dtype=np.int64))
+        acc['nch'].append([chains])
+        lp = np.zeros((nf, 15, 3))
+        lp[:, 1] = rs.normal(0.0, 1.0, size=(nf, 3))
+        acc['lp'].append(lp)
+        acc['lo'].append(_random_so3vec(rs, nf))
+        acc['lt'].append(rs.randint(0, num_fgtype, size=nf))
+        gflag = np.ones(nf, dtype=bool)
+        if gen_mode == 'partial':
+            gflag[: nf // 3] = False
+        acc['gen'].append(gflag)
+        acc['bl'].append(np.full(nf, g))
+        acc['br'].append(np.full(nr, g))
+    cat = lambda k, dt: torch.from_numpy(np.concatenate(acc[k], 0).astype(dt))
+    n_l, n_p = int(sum(n_fg)), int(sum(n_res))
+    batch = {
+        'ligand_pos_heavyatom': cat('lp', np.float32), 'ligand_o_fg': cat('lo', np.float32),
+        'ligand_type_fg': cat('lt', np.int64),
+        'protein_pos_heavyatom': cat('pp', np.float32), 'protein_mask_heavyatom': cat('pm', np.bool_),
+        'protein_aa': cat('aa', np.int64), 'protein_type_fg': cat('aa', np.int64),      # fg_only: type_fg = aa (_base.py:17-27)
+        'protein_res_nb': cat('rnb', np.int64), 'protein_chain_nb': cat('cnb', np.int64),
+        'protein_num_chains': cat('nch', np.int64),
+        'ligand_lig_flag': torch.ones(n_l, dtype=torch.bool), 'protein_lig_flag': torch.zeros(n_p, dtype=torch.bool),
+        'ligand_type_fg_batch': cat('bl', np.int64), 'protein_type_fg_batch': cat('br', np.int64),
+    }
+    if gen_mode == 'partial':
+        batch['ligand_gen_flag'] = cat('gen', np.bool_)
+    return batch
+
+
+def make_d3fg_noise(num_steps, n_fg, num_classes=28, seed=7):
+    """Injected draws of one D3FG.sample call: positions N(0,1) [T,n,3]; rotation {'dir': N(0,1) [T,n,3], 'bin_u' /
+    'in_u': U[0,1) [T,n], 'gauss': N(0,1) [T,n]}; Gumbel uniforms U[0,1) [T,n,K]."""
+    rs = np.random.RandomState(seed)
+    f = lambda a: torch.from_numpy(a.astype(np.float32))
+    pos = f(rs.normal(size=(num_steps, n_fg, 3)))
+    rot = {'dir': f(rs.normal(size=(num_steps, n_fg, 3))), 'bin_u': f(rs.random_sample(size=(num_steps, n_fg))),
+           'in_u': f(rs.random_sample(size=(num_steps, n_fg))), 'gauss': f(rs.normal(size=(num_steps, n_fg)))}
+    return pos, rot, f(rs.random_sample(size=(num_steps, n_fg, num_classes)))
+
+
+# (name, residues per graph, FGs per graph, data seed, gen mode); T = 20, hidden 256, 9 layers, 28 classes
+D3FG_CASES = [
+    ('denovo_ragged', [46, 30, 21], [7, 5, 4], 41, 'denovo'),
+    ('partial', [38, 26], [6, 6], 42, 'partial'),
+    ('below_k', [15], [4], 43, 'denovo'),                 # 19 nodes: fewer than k + 1 = 33
+]
+D3FG_STEPS, D3FG_WEIGHT_SEED, D3FG_NOISE_SEED = 20, 6, 8

@@ -375,6 +375,89 @@ int32_t cbg_ipa_forward_f32(const float* blob, int32_t hidden, int32_t num_subla
                             int32_t k, float* eps_pos, float* h_out, float* o_next, float* r_next, float* logits,
                             void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- D3FG sampler: one reverse step of D3FG.sample (repo/models/diffusion/difffg.py:174-246) per call ------------------
+ * num_classes <= 32 (fg_only mode: 28 FG types).  Per call, on `stream`:
+ *   step-init kernel   composed rows of the ligand FGs: x = x_t, o = o_t and
+ *                        h = (ligand_fg_emb.weight[:, argmax(c_t)] + ligand_fg_emb.bias) + ligand_indicator(1)
+ *                      (argmax = first maximum, like torch.argmax: FGContextEmbedder re-one-hots the 28-wide c_t into its
+ *                      49-wide input, context_emb.py:95-102).  The protein rows of x and o are written once by the caller
+ *                      and never rewritten; those of h are copied from h_static (the layers update h in place).
+ *   IPA encoder        cbg_ipa_forward_f32 on the plan's workspace -> eps_pos, o_pred (gen-masked), logits on every row
+ *   d3fg_reverse       one warp per FG (lane = class), gen_flag-masked (rows without it keep x_t, o_t, argmax(c_t)):
+ *     position  CTNVPScheduler.backward_remove_noise(type='score'):
+ *               x' = (x_t + beta * (-eps / sqrt(1 - alpha_cumprod))) / sqrt(1 - beta) + pos_nonzero * sqrt(beta) * pos_noise
+ *     rotation  RotVPScheduler.backward_remove_noise: e = normalize(rot_dir) * theta if t > 1 else 0,
+ *               o' = log(exp(e) exp(o_pred)) with so3.py's 1e-8 guards and min_cos = -1 (sampling runs without grad);
+ *               theta ~ ApproxAngularDistribution(inverse sigmas) at t:  stddev <= 0.1: |2 sd + sd * rot_gauss| mod pi,
+ *               otherwise X[t, bin] + rot_in_u * (X[t, bin + 1] - X[t, bin]) with the bin drawn below
+ *     type      TypeVPScheduler.backward_remove_noise: log_softmax(logits), the q_v_posterior log-add-exp, Gumbel argmax
+ *               of type_u (categorical.py:26-37)
+ *
+ * Multinomial draw.  The reference draws the histogram bin with torch.multinomial(Y[t, :-1]), whose internal draw cannot
+ * be passed in.  Here a draw is an inverse CDF: with rot_cdf[t] = cumsum(Y[t, :-1]) in float64 (n_bins = 8191 entries
+ * per row, computed once on the host), bin = the first index with rot_cdf[t][bin] > (double)rot_bin_u * rot_cdf[t][n_bins-1].
+ * A bin of zero weight is never chosen, so the distribution is torch.multinomial's; the device searches the same float64
+ * table, so a given uniform selects the same bin as the host definition (oracle/diffusion_fg.py). */
+typedef struct cbg_d3fg_plan {
+  const float* blob;          /* IPA blob (cbg_ipa_* field table) */
+  int32_t hidden;             /* 128 or 256 */
+  int32_t num_sublayers;      /* num_layers * num_x2h */
+  int32_t num_blocks;
+  int32_t num_classes;        /* K <= 32 */
+  int32_t k;                  /* kNN neighbours */
+  const int32_t* graph_ptr;   /* [n_graphs + 1] composed rows */
+  int32_t n_graphs;
+  int32_t max_graph_nodes;
+  int64_t n_nodes;
+  const uint8_t* lig_flag;    /* [n_nodes] composed */
+  const uint8_t* gen_flag;    /* [n_nodes] composed */
+  const int32_t* lig_node;    /* [n_lig] composed row of FG a, increasing */
+  int32_t n_lig;
+  const uint8_t* gen_lig;     /* [n_lig] */
+  const float* fg_wt;         /* [K, hidden] = ligand_fg_emb.weight[:, :K]^T */
+  const float* fg_b;          /* [hidden] ligand_fg_emb.bias */
+  const float* lig_bias;      /* [hidden] ligand_indicator(1) */
+  const float* h_static;      /* [n_nodes, hidden]: the protein rows (h_rec); ligand rows are not read */
+  float* x;                   /* [n_nodes, 3] composed coordinates */
+  float* o;                   /* [n_nodes, 3] composed so3 vectors */
+  const double* rot_cdf;      /* [T, n_bins] */
+  const float* rot_x;         /* [T, n_bins + 1] bin edges (angular_distrib_inv.X) */
+  int32_t n_bins;
+  void* workspace;            /* cbg_d3fg_workspace_bytes, 256-byte aligned */
+  int64_t workspace_bytes;
+} cbg_d3fg_plan;
+
+typedef struct cbg_d3fg_coef {  /* scheduler table entries of step t (host scalars) */
+  float alpha_cumprod;          /* pos_scheduler.alphas_cumprod[t] */
+  float beta;                   /* pos_scheduler.betas[t] */
+  float pos_nonzero;            /* t > 0 */
+  float rot_stddev;             /* rot_scheduler.angular_distrib_inv.stddevs[t] */
+  int32_t rot_approx;           /* angular_distrib_inv.approx_flag[t] */
+  float rot_nonzero;            /* t > 1 */
+  int32_t rot_row;              /* row of rot_cdf / rot_x (= t) */
+  float log_alphas_cumprod_prev;            /* type_scheduler tables at max(t - 1, 0) ... */
+  float log_one_minus_alphas_cumprod_prev;
+  float log_alpha;                          /* ... and at t */
+  float log_one_minus_alpha;
+} cbg_d3fg_coef;
+
+int64_t cbg_d3fg_workspace_bytes(int64_t n_nodes, int32_t hidden, int32_t num_classes);
+int32_t cbg_d3fg_step_f32(const cbg_d3fg_plan* plan, const cbg_d3fg_coef* coef, const float* x_t /*[n_lig,3]*/,
+                          const float* c_t /*[n_lig,K]*/, const float* o_t /*[n_lig,3]*/, const float* pos_noise /*[n_lig,3]*/,
+                          const float* rot_dir /*[n_lig,3]*/, const float* rot_bin_u /*[n_lig]*/,
+                          const float* rot_in_u /*[n_lig]*/, const float* rot_gauss /*[n_lig]*/,
+                          const float* type_u /*[n_lig,K]*/, float* x_next, float* c_next, float* o_next,
+                          int64_t* v_next /*[n_lig]*/, float* eps_pos_out /*[n_lig,3] or NULL*/,
+                          float* logits_out /*[n_lig,K] or NULL*/, float* o_pred_out /*[n_lig,3] or NULL*/, void* stream);
+/* The reverse step alone (test hook, like cbg_reverse_step_f32): eps / logits / o_pred are per-FG rows; bin_out receives
+ * the histogram bin of every row (drawn whether or not the Gaussian branch is taken), or NULL. */
+int32_t cbg_d3fg_reverse_f32(const cbg_d3fg_coef* coef, const double* rot_cdf, const float* rot_x, int32_t n_bins,
+                             const float* eps /*[n,3]*/, const float* logits /*[n,K]*/, const float* o_pred /*[n,3]*/,
+                             const float* x_t, const float* c_t, const float* o_t, const uint8_t* gen,
+                             const float* pos_noise, const float* rot_dir, const float* rot_bin_u, const float* rot_in_u,
+                             const float* rot_gauss, const float* type_u, int32_t n, int32_t num_classes, float* x_next,
+                             float* c_next, float* o_next, int64_t* v_next, int32_t* bin_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
